@@ -2,7 +2,7 @@
 """bench.py - separator frames/sec on B200 (BASELINE.json metric), one JSON line on stdout.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload c2|c4|c5|c1] [--model NAME] [--seconds S] [--batch B]
+                    [--workload c2|c4|c5|c1] [--model NAME] [--seconds S] [--batch B] [--dump-outputs DIR]
 
 Workloads (BASELINE.json configs, SURVEY.md 8d; weights are seeded random values of the real architecture - the
 reference checkpoint is a Git-LFS pointer, SURVEY.md F3 - hence `"data": "synthetic"`):
@@ -19,9 +19,14 @@ A "step" is one separator forward over the per-GPU batch.
                the library on the launching stream; plus whole-step tensor and HBM fractions
   parity       checked on the TIMED configuration: two utterances of the timed batch against the fp32 CUDA-core path,
                finiteness of the whole output, and the SI-SNRi delta against the CPU oracle on a short mixture
-  reference_gpu  the reference's own Separator (baseline/_ref, eager PyTorch) on the same B200, fp32 and allow_tf32
-  cpu_baseline / --impl reference: the reference's Separator (baseline/_ref; else its restatement in oracle/) on the
+  reference_gpu  the reference's own Separator (oracle/_ref, eager PyTorch) on the same B200, fp32 and allow_tf32
+  cpu_baseline / --impl reference: the reference's Separator (oracle/_ref; else its restatement in oracle/) on the
                host cores
+
+--dump-outputs DIR writes what the last timed step returned (the separator's last-stage output and its per-stage outputs)
+as DIR/<name>.npy, float32; arrays too large for a 60 MB budget are sampled at fixed seeded positions, and
+DIR/manifest.json records each array's shape and whether it was sampled.  The inputs depend on the arguments alone, so
+two builds can be compared output for output.  (--impl reference times the CPU reference and has no outputs to dump.)
 
 N > 1: launched by torch.distributed.run, one rank per GPU; utterances shard (weak scaling); the only collective is an
 all-gather of the per-utterance metric vector, inside the timed region as the last thing each step does.
@@ -46,7 +51,8 @@ WORKLOADS = {
     "c5": dict(model="SepReformer_Large_DM_WSJ0", samples=80000, batch=8, tag="configs[4] per GPU"),
     "c1": dict(model="SepReformer_Base_WSJ0", samples=73596, batch=1, tag="configs[0] shape (sample_WSJ.wav length)"),
 }
-REF_COPY = os.path.join(ROOT, "baseline", "_ref")
+REF_COPY = os.path.join(ROOT, "oracle", "_ref")
+DUMP_BYTES = 60 << 20
 
 
 def frames_of(samples):
@@ -137,7 +143,7 @@ def seeded_separator_state(model):
 
 
 def reference_separator(model):
-    """The reference's own Separator (unmodified files under baseline/_ref, tools/install_reference.py) with the seeded
+    """The reference's own Separator (unmodified files under oracle/_ref, oracle/install_reference.py) with the seeded
     weights loaded; None when the copy is not there."""
     if not os.path.isdir(os.path.join(REF_COPY, "models", model)):
         return None
@@ -156,7 +162,7 @@ def reference_separator(model):
 
 
 def cpu_forward_fn(model, x):
-    """(callable, kind): the reference Separator on the CPU when baseline/_ref is present, else the oracle port."""
+    """(callable, kind): the reference Separator on the CPU when oracle/_ref is present, else the oracle port."""
     ref = reference_separator(model)
     if ref is not None:
         return (lambda: ref(x)), "reference"
@@ -218,13 +224,13 @@ def run_reference(args, wl):
         return
     model, samples = wl["model"], wl["samples"]
     batch = 1
-    steps = min(args.steps, 5)          # bounded CPU sample
-    r = time_cpu(model, samples, batch, steps, 1)
-    what = ("the reference's own Separator (unmodified files, baseline/_ref)" if r["kind"] == "reference"
-            else "oracle/ restatement of the reference Separator (baseline/_ref not present)")
+    steps = args.steps
+    r = time_cpu(model, samples, batch, steps, args.warmup)
+    what = ("the reference's own Separator (unmodified files, oracle/_ref)" if r["kind"] == "reference"
+            else "oracle/ restatement of the reference Separator (oracle/_ref not present)")
     line = {
         "impl": "reference", "metric": "separator frames/sec", "value": r["fps"], "unit": "frames/s", "n_gpus": args.gpus,
-        "steps": steps, "warmup": 1, "ms_per_step": r["ms"], "higher_is_better": True,
+        "steps": steps, "warmup": args.warmup, "ms_per_step": r["ms"], "higher_is_better": True,
         "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": f"{model} separator forward, {samples} samples @ 8 kHz 2-spk ({frames_of(samples)} frames/utt), "
                                f"CPU sample of {batch} utterance per step", "global_batch": batch, "frames_per_utt": frames_of(samples)},
@@ -239,7 +245,7 @@ def run_reference(args, wl):
 
 def time_reference_on_gpu(model, x_dev, steps=3):
     """SURVEY.md 8d / BASELINE.md 3: the reference Separator itself, eager PyTorch on this B200 (the honest GPU
-    baseline): fp32, and again with TF32 matmuls allowed.  Returns None when baseline/_ref is absent."""
+    baseline): fp32, and again with TF32 matmuls allowed.  Returns None when oracle/_ref is absent."""
     ref = reference_separator(model)
     if ref is None:
         return None
@@ -266,9 +272,29 @@ def time_reference_on_gpu(model, x_dev, steps=3):
         torch.backends.cudnn.allow_tf32 = True
     del ref
     torch.cuda.empty_cache()
-    out["what"] = ("reference Separator (baseline/_ref, unmodified), eager PyTorch on this GPU, inference_mode, same batch and "
+    out["what"] = ("reference Separator (oracle/_ref, unmodified), eager PyTorch on this GPU, inference_mode, same batch and "
                    f"weights, {steps} timed forwards after 2 warm-ups, CUDA events")
     return out
+
+
+def dump_outputs(outdir, arrays):
+    """Each array as <outdir>/<name>.npy in float32; one larger than its share of DUMP_BYTES is replaced by the elements at
+    a seeded, sorted set of flat (row-major) positions, the same positions for the same shape on every run.
+    <outdir>/manifest.json gives, per name, the array's shape and, when sampled, the seed and sample size."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    cap = DUMP_BYTES // 4 // len(arrays)
+    manifest = {}
+    for name, t in arrays.items():
+        a = t.detach().float()
+        manifest[name] = {"shape": list(a.shape), "dtype": "float32", "sampled": a.numel() > cap}
+        if a.numel() > cap:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:cap].sort().values
+            a = a.reshape(-1)[idx.to(a.device)]
+            manifest[name].update(sample="torch.randperm(numel, Generator().manual_seed(0))[:n].sort()", seed=0, n=cap)
+        np.save(os.path.join(outdir, name + ".npy"), a.cpu().numpy())
+    with open(os.path.join(outdir, "manifest.json"), "w") as f:
+        json.dump(manifest, f, indent=1)
 
 
 # ------------------------------------------------------------------------------------------------ parity on the timed config
@@ -367,7 +393,9 @@ def run_ours(args, wl):
     mix_host = (s1 + s2).pin_memory()
     mix_dev = mix_host.to(dev)
     tgt_dev = torch.stack([s1, s2]).to(dev)
-    with torch.no_grad():                # separator input exactly as this model's shell produces it (module.py:12-35)
+    # separator input exactly as this model's shell produces it (module.py:12-35); deterministic convolutions, so the
+    # same arguments give the same input on every run
+    with torch.no_grad(), torch.backends.cudnn.flags(enabled=True, deterministic=True):
         e = torch.nn.functional.gelu(model.audio_encoder.conv1d(mix_dev[:, None]))
         x_dev = model.feature_projector.conv1d(model.feature_projector.norm(e)).contiguous()
         del e
@@ -381,11 +409,11 @@ def run_ours(args, wl):
     from sepreformer_b200.sharding import gather_utterance_values
 
     def step_device():
-        last, _ = sep(x_dev)
+        out = sep(x_dev)
         if world > 1:     # the path's only exchange (SURVEY 8e): per-utterance PIT SI-SNRi rows [B_local, 3], computed on the
             # device (k_pit_sisnri), all-gathered into global utterance order on every rank
             gather_utterance_values(model.pit_si_snri(audio_dev, tgt_dev, mix_dev), B * world)
-        return last
+        return out
 
     def barrier():
         if world > 1:
@@ -403,12 +431,15 @@ def run_ours(args, wl):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(args.steps):
-            last_timed = step_device()
+            last_timed, stages_timed = step_device()
         e1.record()
         barrier()
         ms_total = e0.elapsed_time(e1)
         launches = sep.last_launch_count * args.steps
         clk = clocks.stop() if rank == 0 else None
+        if args.dump_outputs and rank == 0:      # before any other call reuses the graph's output buffers
+            dump_outputs(args.dump_outputs, {"last": last_timed, **{f"stage{i}": t for i, t in enumerate(stages_timed)}})
+        del stages_timed
 
         # ---- the timed configuration is checked (rank 0; after the timed region)
         parity = parity_block(sep, x_dev, last_timed, model_name, args.no_cpu_baseline) if rank == 0 else None
@@ -549,7 +580,7 @@ def run_ours(args, wl):
                 "value": cpu["fps"], "unit": "frames/s", "cores": cpu["threads"], "kind": cpu["kind"],
                 "sample": f"2 timed forwards of 1 utterance of the same synthetic workload on the host cores ({cpu_model_name()}, "
                           f"{cpu['logical_cores']} logical), {cpu['threads']} threads (proxy seconds by thread count {cpu['proxy_s']}); "
-                          + ("reference Separator from baseline/_ref" if cpu["kind"] == "reference" else "oracle/ restatement")},
+                          + ("reference Separator from oracle/_ref" if cpu["kind"] == "reference" else "oracle/ restatement")},
             "reference_gpu": ref_gpu,
             "host_enqueue_ms_b1": host_ms_b1,
             "kernel_ms": prof,
@@ -574,7 +605,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help="skip the CPU legs (oracle SI-SNRi check and cpu_baseline)")
     ap.add_argument("--no-reference-gpu", action="store_true", help="skip timing the reference Separator on the GPU")
     ap.add_argument("--no-cuda-graph", action="store_true", help="launch every kernel individually (SEPREF_OPT_CUDA_GRAPH off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (float32, seeded sample above 60 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs applies to --impl ours: the reference arm times the CPU reference and returns nothing")
     wl = WORKLOADS[args.workload]
     if args.model or args.seconds or args.batch:
         wl = dict(wl)

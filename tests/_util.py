@@ -8,14 +8,13 @@ from sepreformer_b200.configs import MODEL_SHAPES
 from sepreformer_b200.params import ParamTree, separator_spec, seeded_state, state_shapes
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-HAVE_REFERENCE = os.path.isdir("/root/reference/models")
-# the runnable copy of the reference's model files (tools/install_reference.py; git-ignored, ships to the GPU box)
-REF_COPY = os.path.join(os.path.dirname(GOLDEN.rstrip("/")).rsplit("/tests", 1)[0], "baseline", "_ref")
-REF_DIR = "/root/reference" if HAVE_REFERENCE else (REF_COPY if os.path.isdir(os.path.join(REF_COPY, "models")) else None)
+# the runnable copy of the reference's model files (oracle/install_reference.py, run by build(); git-ignored)
+REF_COPY = os.path.join(os.path.dirname(os.path.dirname(GOLDEN)), "oracle", "_ref")
+REF_DIR = REF_COPY if os.path.isdir(os.path.join(REF_COPY, "models")) else None
 
 
 def reference_model_module(name):
-    """Import ``models.<name>.model`` of the reference (from /root/reference or baseline/_ref) with its logger silenced."""
+    """Import ``models.<name>.model`` of the reference (from oracle/_ref) with its logger silenced."""
     import importlib
     import sys
     if REF_DIR is None:

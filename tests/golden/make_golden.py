@@ -1,8 +1,10 @@
 """Generate the golden vectors under tests/golden/ by running the *reference itself*.
 
-Run in the build container only (needs /root/reference; the GPU box has neither it nor this need):
+Needs a checkout of the original SepReformer project (github.com/dmlguq456/SepReformer), found as
+oracle/install_reference.py finds it (``SEPREFORMER_REFERENCE``, else ``/root/reference``); the tests only read what
+this writes:
 
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py [case ...]
 
 For every case the reference ``Separator`` (or one of its block classes) is instantiated from the
 reference's own configs.yaml, loaded (strict) with ``sepreformer_b200.params.seeded_state(seed)`` -
@@ -20,8 +22,9 @@ import yaml
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-sys.path.insert(0, "/root/reference")
 sys.path.insert(0, ROOT)
+from oracle.install_reference import SRC as REF  # noqa: E402
+sys.path.insert(0, REF)
 
 from loguru import logger  # noqa: E402
 
@@ -43,7 +46,7 @@ def checksums(sd):
 
 def ref_separator(model_name):
     mod = importlib.import_module(f"models.{model_name}.modules.module")
-    cfg = yaml.full_load(open(f"/root/reference/models/{model_name}/configs.yaml"))["config"]["model"]["module_separator"]
+    cfg = yaml.full_load(open(os.path.join(REF, "models", model_name, "configs.yaml")))["config"]["model"]["module_separator"]
     return mod.Separator(**cfg).eval(), mod
 
 
@@ -100,7 +103,100 @@ def block_cases(tag, model_name, wseed, xseed, batch=2, td=3):
     print(tag, {k: v.shape for k, v in out.items() if hasattr(v, "shape") and v.ndim > 1})
 
 
+def _ref_model(model_name):
+    cfg = yaml.full_load(open(os.path.join(REF, "models", model_name, "configs.yaml")))["config"]["model"]
+    return importlib.import_module(f"models.{model_name}.model").Model, cfg
+
+
+def _strided(out, key, t, stride, dtype):
+    out[key] = t[..., ::stride].to(dtype).numpy()
+    out[key + "_norm"] = float(t.double().norm())
+
+
+def model_shell_case(tag, stride=4):
+    """tests/test_model_shell.py: the reference Model in fp64 with the oracle's seeded shell weights."""
+    from _util import model_state, seeded_input
+    from test_model_shell import shell_state
+    Model, cfg = _ref_model("SepReformer_Base_WSJ0")
+    ref = Model(**cfg).eval()
+    ref.separator.load_state_dict(model_state("SepReformer_Base_WSJ0", 7), strict=True)
+    missing, unexpected = ref.load_state_dict(shell_state(), strict=False)
+    assert not unexpected and all(not k.startswith(("audio_encoder", "feature_projector", "out_layer.", "audio_decoder")) for k in missing)
+    ref = ref.double()
+    mix = 0.1 * seeded_input(9, 2, 4000).double()
+    with torch.no_grad():
+        audio, _ = ref(mix)
+    out = dict(stride=stride)
+    for s, a in enumerate(audio):
+        _strided(out, f"audio{s}", a, stride, torch.float64)
+    np.savez_compressed(os.path.join(HERE, tag + ".npz"), **out)
+    print(tag, [a.shape for a in audio])
+
+
+def pit_criterion_case(tag):
+    """tests/test_model_shell.py: the reference's PIT_SISNRi (utils/implements/criterions.py) on three seeded trials;
+    the two packages it imports but this path never touches are stubbed."""
+    import types
+    for missing in ("mir_eval", "mir_eval.separation", "torchaudio", "torchaudio.transforms"):
+        if missing not in sys.modules:
+            try:
+                __import__(missing)
+            except Exception:
+                mod = types.ModuleType(missing)
+                mod.bss_eval_sources = None
+                mod.MelScale = object
+                sys.modules[missing] = mod
+    from utils.implements.criterions import PIT_SISNRi
+    from test_model_shell import pit_trials
+    crit = PIT_SISNRi(device=torch.device("cpu"), num_spks=2, scale_inv=True)
+    vals = []
+    for e, (s1, s2), mix in pit_trials():
+        v, _ = crit(estims=e, mixture=mix, input_sizes=torch.tensor([mix.shape[-1]]), target_attr=[s1, s2], eps=1.0e-15)
+        vals.append(float(v))
+    np.savez_compressed(os.path.join(HERE, tag + ".npz"), pit_sisnri=np.array(vals))
+    print(tag, vals)
+
+
+def separator_fp64_case(tag, stride=8):
+    """tests/test_oracle_golden.py: the reference Separator in fp64, stored in fp64 (compared at 1e-12)."""
+    from _util import model_state
+    ref, _ = ref_separator("SepReformer_Base_WSJ0")
+    ref.load_state_dict(model_state("SepReformer_Base_WSJ0", 7), strict=True)
+    ref = ref.double()
+    x = seeded_input(5, 1, 128, 203).double()
+    with torch.no_grad():
+        last, stages = ref(x)
+    out = dict(stride=stride)
+    _strided(out, "last", last, stride, torch.float64)
+    for i, s in enumerate(stages):
+        _strided(out, f"stage{i}", s, stride, torch.float64)
+    np.savez_compressed(os.path.join(HERE, tag + ".npz"), **out)
+    print(tag, last.shape, [s.shape for s in stages])
+
+
+def model_level_case(tag, model_name="SepReformer_Base_WSJ0", stride=16):
+    """tests/test_model_gpu.py: the stock reference Model in fp32 with every entry of its state_dict seeded
+    (``seeded_state`` in state_dict order), on the seeded mixtures of that test; audio and the four auxiliary heads."""
+    import json
+    from test_model_gpu import mixtures
+    Model, cfg = _ref_model(model_name)
+    ref = Model(**cfg).eval()
+    ref.load_state_dict(seeded_state(state_shapes(ref), seed=1), strict=True)
+    mix, _, _ = mixtures(2, 8000)
+    with torch.inference_mode():
+        audio, aux = ref(mix)
+    out = dict(model=np.array(model_name), cfg=np.array(json.dumps(cfg)), keys=np.array(list(ref.state_dict())), stride=stride)
+    for s, a in enumerate(audio):
+        _strided(out, f"audio{s}", a, stride, torch.float32)
+    for i, heads in enumerate(aux):
+        for s, a in enumerate(heads):
+            _strided(out, f"aux{i}_{s}", a, stride, torch.float32)
+    np.savez_compressed(os.path.join(HERE, tag + ".npz"), **out)
+    print(tag, audio[0].shape, len(aux))
+
+
 if __name__ == "__main__":
+    sys.path.insert(0, os.path.dirname(HERE))      # the tests' helpers, for the cases that mirror a test
     only = set(sys.argv[1:])        # optional: regenerate just the named cases
 
     def separator_case(tag, *a, _f=separator_case, **k):      # noqa: F811
@@ -120,3 +216,7 @@ if __name__ == "__main__":
     separator_case("sep_large_medium", "SepReformer_Large_DM_WSJ0", batch=1, t_enc=2003, wseed=5, xseed=16, stride=8)
     block_cases("blocks_base", "SepReformer_Base_WSJ0", wseed=1, xseed=21)
     block_cases("blocks_large", "SepReformer_Large_DM_WSJ0", wseed=5, xseed=22)
+    for tag, case in (("model_shell_base", model_shell_case), ("pit_criterion", pit_criterion_case),
+                      ("sep_base_fp64", separator_fp64_case), ("model_base", model_level_case)):
+        if not only or tag in only:
+            case(tag)

@@ -1,6 +1,6 @@
 """The model-level path (SURVEY.md 8f rows n1-n4): waveform -> AudioEncoder/FeatureProjector -> separator -> OutputLayer ->
 AudioDecoder -> waveforms in ONE C-ABI call (sepref_model_forward), against the CPU oracle's model shell (pinned to the
-reference Model in test_model_shell.py), the reference Model itself where its files are shipped, and the device-side
+reference Model in test_model_shell.py), the reference Model itself through golden vectors, and the device-side
 batched PIT SI-SNRi against the oracle's restatement of criterions.py:221-260."""
 import pytest
 import torch
@@ -10,7 +10,7 @@ from oracle import separator_oracle as O
 from sepreformer_b200 import MODEL_SHAPES, separator_kwargs
 from sepreformer_b200.params import seeded_state, state_shapes
 
-from _util import REF_DIR, reference_model_config, reference_model_module, rel_l2
+from _util import load_golden, rel_l2
 
 pytestmark = pytest.mark.gpu
 
@@ -129,35 +129,33 @@ def test_si_snri_delta_through_the_model_path():
     assert delta <= 0.05
 
 
-@pytest.mark.skipif(REF_DIR is None, reason="reference files not shipped (tools/install_reference.py)")
 def test_model_level_install_matches_reference_model_including_aux_heads():
-    name = "SepReformer_Base_WSJ0"
-    mm = reference_model_module(name)
-    cfg = reference_model_config(name)
-    stock = mm.Model
-    torch.manual_seed(0)
-    ref = stock(**cfg).eval()
-    ref.separator.load_state_dict(seeded_state(state_shapes(ref.separator), seed=1), strict=True)
-    try:
-        sepreformer_b200.install(mm, level="model")
-        ours = mm.Model(**cfg)
-    finally:
-        mm.Model = stock
+    """install(level="model") against the stock reference Model (tests/golden/make_golden.py): same state_dict keys in
+    the same order, and the same audio and auxiliary-head outputs on the same seeded weights and mixtures."""
+    import json
+    import types
+    gold = load_golden("model_base")
+    st = int(gold["stride"])
+    cfg = json.loads(str(gold["cfg"]))
+    mm = sepreformer_b200.install(types.ModuleType("model"), level="model")
+    ours = mm.Model(**cfg)
     assert isinstance(ours, sepreformer_b200.Model)
+    assert list(ours.state_dict()) == [str(k) for k in gold["keys"]]
+    sd = seeded_state(state_shapes(ours), seed=1)
     ours = ours.cuda().eval()
-    ours.load_state_dict(ref.state_dict(), strict=True)          # AFTER .cuda(): the load hook must re-pack the weights
+    ours.load_state_dict(sd, strict=True)          # AFTER .cuda(): the load hook must re-pack the weights
     mix, _, _ = mixtures(2, 8000)
     with torch.inference_mode():
-        want, want_aux = ref(mix)
         got, got_aux = ours(mix.cuda())
     for s in range(2):
-        err = rel_l2(got[s].cpu(), want[s])
+        err = rel_l2(got[s].cpu()[..., ::st], gold[f"audio{s}"])
         print(f"model-level install, speaker {s}: rel-L2 {err:.2e}")
-        assert err < 1e-3
-    assert len(got_aux) == len(want_aux) == 4
-    for a, b in zip(got_aux, want_aux):
+        assert got[s].shape[-1] == mix.shape[-1] and err < 1e-3
+    assert len(got_aux) == 4
+    for i, heads in enumerate(got_aux):
         for s in range(2):
-            assert a[s].shape == b[s].shape and rel_l2(a[s].cpu(), b[s]) < 1e-3
+            want = gold[f"aux{i}_{s}"]
+            assert heads[s][..., ::st].shape == want.shape and rel_l2(heads[s].cpu()[..., ::st], want) < 1e-3
 
 
 def test_cuda_graph_replay_is_bit_identical_and_cheap_to_enqueue():

@@ -1,11 +1,11 @@
-"""Pin the CPU oracle to the reference: golden vectors (always) and the live reference (when mounted)."""
+"""Pin the CPU oracle to the reference through golden vectors made by tests/golden/make_golden.py."""
 import pytest
 import torch
 
 from oracle import separator_oracle as O
 from sepreformer_b200.configs import MODEL_SHAPES
 
-from _util import (HAVE_REFERENCE, check_generator_stable, load_golden, model_state, rel_l2, seeded_input)
+from _util import check_generator_stable, load_golden, model_state, rel_l2, seeded_input
 
 SEP_CASES = ["sep_base_small", "sep_base_exact16", "sep_base_medium", "sep_large_whamr_small", "sep_large_wham_small",
              "sep_large_medium"]
@@ -102,24 +102,16 @@ def test_pit_sisnri_permutation_invariant():
     assert torch.allclose(a, b) and float(a.min()) > 15.0
 
 
-@pytest.mark.skipif(not HAVE_REFERENCE, reason="live reference only exists in the build container")
 def test_oracle_matches_live_reference():
-    import importlib
-    import sys
-    import yaml
-    sys.path.insert(0, "/root/reference")
-    from loguru import logger
-    logger.remove()
-    name = "SepReformer_Base_WSJ0"
-    mod = importlib.import_module(f"models.{name}.modules.module")
-    cfg = yaml.full_load(open(f"/root/reference/models/{name}/configs.yaml"))["config"]["model"]["module_separator"]
-    ref = mod.Separator(**cfg).eval()
-    sd = model_state(name, 7)
-    ref.load_state_dict(sd, strict=True)
-    ref = ref.double()
+    """The reference Separator's fp64 output, stored in fp64: agreement to 1e-12, not just float32 rounding."""
+    gold = load_golden("sep_base_fp64")
+    st = int(gold["stride"])
+    sd = model_state("SepReformer_Base_WSJ0", 7)
     x = seeded_input(5, 1, 128, 203).double()
     with torch.no_grad():
-        yr, sr = ref(x)
         yo, so = O.separator_forward(x, {k: v.double() for k, v in sd.items() if v.is_floating_point()})
-    assert rel_l2(yo, yr) < 1e-12
-    assert all(rel_l2(a, b) < 1e-12 for a, b in zip(so, sr))
+    assert len(so) == sum(k.startswith("stage") and not k.endswith("_norm") for k in gold)
+    for key, t in [("last", yo)] + [(f"stage{i}", s) for i, s in enumerate(so)]:
+        assert t[..., ::st].shape == gold[key].shape, key
+        assert rel_l2(t[..., ::st], gold[key]) < 1e-12, key
+        assert abs(float(t.norm()) - float(gold[key + "_norm"])) < 1e-12 * float(gold[key + "_norm"]), key
